@@ -522,3 +522,101 @@ def test_host_enqueued_and_plain_launch_paths_give_the_same_fit(env, tmp_path, m
     assert v["trips"].tolist() == est.n_iter_.tolist() == g["trips"].tolist()
     assert int(v["graph"]) == (0 if "TPLS_NO_GRAPH" in env else 1)
     assert np.array_equal(v["T"], est.factor_T) and np.array_equal(v["coef"], est.coef_)
+
+
+# ---------------------------------------------------------------------------
+# transform and reconstruction at sizes where the rings of multiproj_kernel and the reconstruction's bounce buffers
+# cycle, against the oracle / numpy on a random model (unit-norm loadings, a mean of order 1, data = mean + noise)
+# ---------------------------------------------------------------------------
+def _random_model(shapes, R, dtypes, seed):
+    rng = np.random.default_rng(seed)
+    Xs, means, loadings = [], [], []
+    for shape, dt in zip(shapes, dtypes):
+        ws = [rng.normal(size=(d, R)) for d in shape[1:]]
+        loadings.append([w / np.linalg.norm(w, axis=0) for w in ws])
+        mu = rng.normal(size=shape[1:]).astype(dt)
+        means.append(mu)
+        Xs.append((mu + rng.normal(size=shape)).astype(dt))
+    return Xs, means, loadings
+
+
+# multiproj_kernel (multiproj.cu): 16-row tiles through a 3-stage ring, one CTA per (row block, column slab) with
+# 148 / n_slabs CTAs per slab.  40001 rows = 2501 tiles, the last one 1 row, so CTAs run different numbers of laps.
+_TRANSFORM_CASES = [
+    # (64, 64) fp32: NB = 1, 2 -> 8 slabs of 512, 18 CTAs per slab x 138-139 tiles = 46-47 laps
+    ([(40001, 64, 64)], 3, [np.float32]),
+    ([(40001, 64, 64)], 10, [np.float32]),
+    # NB = 3, 4 -> half-width slabs: 16 slabs of 256, 9 CTAs per slab x 277-278 tiles
+    ([(40001, 64, 64)], 17, [np.float32]),
+    ([(40001, 64, 64)], 32, [np.float32]),
+    # fp64, NB = 2: 16 slabs of 256 columns, 9 CTAs per slab
+    ([(40001, 64, 64)], 10, [np.float64]),
+    # P = 5200: 11 slabs, the last one 80 columns wide, 13 CTAs per slab x 192-193 tiles
+    ([(40001, 130, 40)], 10, [np.float32]),
+    # odd P = 561 in fp64: pitched staging copy (pitch 562), 3 slabs (256, 256, 50), 49 CTAs per slab x 51-52 tiles
+    ([(40001, 33, 17)], 5, [np.float64]),
+    # a coupled pair with different P: 8 slabs + 1 slab (148 CTAs x 16-17 tiles), both summed by multiproj_finish
+    ([(40001, 64, 64), (40001, 24, 20)], 10, [np.float32, np.float32]),
+]
+
+
+@pytest.mark.parametrize("shapes,R,dtypes", _TRANSFORM_CASES)
+def test_transform_at_size_matches_oracle(shapes, R, dtypes):
+    """Complete data: the single-pass path (all R projections in one read of X, then the score recurrence) computes
+    in fp64 on the stored values and never rounds a deflated value -> 1e-10 per column against the oracle's sequential
+    project/deflate in fp64, for host input and for torch CUDA input read in place.  With one NaN in the last tile
+    and one all-NaN row the sequential masked path runs instead (deflated values rounded to the stored dtype)."""
+    import torch
+    from oracle import tpls_oracle as orc
+    from cmtf_pls_b200 import _core
+    Xs, means, loadings = _random_model(shapes, R, dtypes, seed=sum(s[1] for s in shapes) + R)
+    state = {"T": np.empty((0, R)), "X_mean": [m.astype(np.float64) for m in means], "W": loadings}
+    want = orc.transform(state, [x.astype(np.float64) for x in Xs])
+    eng = _core.get_engine(0)
+    for kind in ("host", "cuda"):
+        arg = Xs if kind == "host" else [torch.from_numpy(x).cuda() for x in Xs]
+        got = _core.run_transform(arg, means, loadings, R)
+        assert eng.stats()["last_transform_path"] == 1, kind
+        assert col_err(got, want) < 1e-10, (kind, col_err(got, want))
+        del arg
+    del want
+    n = shapes[0][0]
+    Xm = [x.copy() for x in Xs]
+    del Xs
+    Xm[-1][n - 1].reshape(-1)[-1] = np.nan        # one NaN in the last row (the 1-row last tile)
+    Xm[0][n // 2] = np.nan                        # one row entirely NaN: NaN scores, like the reference
+    got = _core.run_transform(Xm, means, loadings, R)
+    assert eng.stats()["last_transform_path"] == 2
+    want = orc.transform(dict(state, X_mean=means), Xm)         # on the stored dtype, as the masked path computes
+    assert np.array_equal(np.isnan(got), np.isnan(want))
+    assert np.isnan(got[n // 2]).all() and np.isnan(got).sum() == R
+    keep = ~np.isnan(want[:, 0])
+    tol = FP32_TOL if np.float32 in dtypes else FP64_TOL
+    assert col_err(got[keep], want[keep]) < tol
+
+
+# tpls_reconstruct with a host result: blocks of 32 MiB / (8 p) rows through two device blocks and two pinned bounce
+# buffers.  n = 5000, p = 4096: 1024-row blocks, 5 of them, the last 904 rows, so both buffers cycle; p = 5200: 806-row
+# blocks, 7 of them, the last 164 rows.
+@pytest.mark.parametrize("p", [4096, 5200])
+@pytest.mark.parametrize("R", [1, 32])
+@pytest.mark.parametrize("mean_dtype", [np.float32, np.float64])
+def test_reconstruct_host_blocks_match_numpy(p, R, mean_dtype):
+    import torch
+    from cmtf_pls_b200 import _core
+    from cmtf_pls_b200._engine import dtype_code
+    rng = np.random.default_rng(p + R)
+    n = 5000
+    scores = rng.normal(size=(n, R))
+    wkron = rng.normal(size=(R, p)) / np.sqrt(p)
+    mean = rng.normal(size=p).astype(mean_dtype)
+    eng = _core.get_engine(0)
+    got = eng.reconstruct(scores, wkron, mean)
+    want = scores @ wkron + mean.astype(np.float64)
+    assert got.shape == (n, p) and np.max(np.abs(got - want)) <= 1e-12 * np.max(np.abs(want))
+    # the device-result branch (one launch over all rows) computes every element the same way: bit for bit
+    out = torch.empty((n, p), dtype=torch.float64, device="cuda")
+    eng._ck(eng.lib.tpls_reconstruct(eng.h, R, scores.ctypes.data, n, p, wkron.ctypes.data, mean.ctypes.data,
+                                     dtype_code(mean), out.data_ptr()))
+    assert np.array_equal(out.cpu().numpy(), got)
+
