@@ -11,6 +11,7 @@ include/tpls_b200.h.  There is no CPU fallback.
 from .tpls import tPLS
 from .cmtf import ctPLS
 from .validate import get_q2y, q2y_sweep
+from .batch import fit_batch
 
 
 
@@ -24,4 +25,4 @@ def trim_memory():
 
 
 __version__ = "0.1.0"
-__all__ = ["tPLS", "ctPLS", "get_q2y", "q2y_sweep", "trim_memory"]
+__all__ = ["tPLS", "ctPLS", "fit_batch", "get_q2y", "q2y_sweep", "trim_memory"]

@@ -23,6 +23,7 @@ FIT_PROFILE = 2
 FIT_COVARIANCE = 4
 MAX_TENSORS = 8
 MAX_MODES = 8
+E_BATCH_UNSUPPORTED = 2   # tpls_fit_batch: a problem is outside the batch kernel's limits, nothing was written
 
 _lib = None
 
@@ -56,6 +57,25 @@ KERNEL_CLASSES = ["colstat", "contract", "project", "deflate_contract", "residua
 
 class Profile(C.Structure):
     _fields_ = [("ms", C.c_double * 10), ("launches", C.c_int64 * 10), ("bytes", C.c_double * 10)]
+
+
+class BatchOut(C.Structure):
+    """Mirror of ``tpls_batch_out``: caller-owned results of ``tpls_fit_batch``, leading axis = problem."""
+    _fields_ = [
+        ("T", C.c_void_p),
+        ("U", C.c_void_p),
+        ("Q", C.c_void_p),
+        ("W", C.c_void_p * MAX_TENSORS),
+        ("coef", C.c_void_p),
+        ("r2x", C.c_void_p),
+        ("r2y", C.c_void_p),
+        ("x_mean", C.c_void_p * MAX_TENSORS),
+        ("y_mean", C.c_void_p),
+        ("trips", C.c_void_p),
+        ("converged", C.c_void_p),
+        ("has_missing", C.c_void_p),
+        ("fit_ms", C.c_double),
+    ]
 
 
 # name -> (restype, argtypes); every symbol declared in include/tpls_b200.h
@@ -92,6 +112,9 @@ SIGNATURES = {
     "tpls_transform": (C.c_int, [_H, C.c_int, C.c_int, C.POINTER(_P), C.POINTER(C.c_int), C.c_int64,
                                  C.POINTER(C.c_int64), C.POINTER(_P), C.POINTER(_P), _P, _P, _P]),
     "tpls_reconstruct": (C.c_int, [_H, C.c_int, _P, C.c_int64, C.c_int64, _P, _P, C.c_int, _P]),
+    "tpls_fit_batch": (C.c_int, [_H, C.c_int, C.c_int64, C.POINTER(_P), C.POINTER(C.c_int), C.POINTER(C.c_int),
+                                 C.POINTER(C.POINTER(C.c_int64)), C.POINTER(C.c_int64), _P, C.c_int64, C.c_int64, _P,
+                                 C.c_int, C.c_double, C.c_int, C.c_int, C.POINTER(BatchOut)]),
     "tpls_op_contract": (C.c_int, [_H, _P, C.c_int, C.c_int64, C.c_int64, _P, C.c_int, _P, C.POINTER(C.c_float), C.c_int]),
     "tpls_op_project": (C.c_int, [_H, _P, C.c_int, C.c_int64, C.c_int64, _P, C.c_int, _P, C.POINTER(C.c_float), C.c_int]),
     "tpls_op_deflate_contract": (C.c_int, [_H, _P, C.c_int, C.c_int64, C.c_int64, _P, _P, _P, C.c_int, _P, _P,
@@ -216,6 +239,25 @@ class Engine:
             self._ck(self.lib.tpls_fit(self.h, n_tensors, n_components, float(tol), int(max_iter), flags))
         finally:
             self._keep.clear()   # the staged inputs are not pinned by a failed fit either
+
+    def fit_batch(self, batch, xs, x_strides, shapes, y, y_stride, m, row_w, n_components, tol, max_iter, out, flags=0):
+        """tpls_fit_batch.  xs / y / row_w: numpy arrays or torch tensors (host or CUDA) with the problems at the
+        given element strides; ``shapes`` the per-problem shapes (n, d1, ...); ``out`` a filled BatchOut.  Returns
+        True when the batch kernel ran, False on E_BATCH_UNSUPPORTED (nothing written); raises on errors."""
+        L = len(xs)
+        ptrs = (_P * L)(*[_ptr(x) for x in xs])
+        dts = (C.c_int * L)(*[dtype_code(x) for x in xs])
+        nds = (C.c_int * L)(*[len(s) for s in shapes])
+        shp = [(C.c_int64 * len(s))(*[int(v) for v in s]) for s in shapes]
+        shps = (C.POINTER(C.c_int64) * L)(*[C.cast(a, C.POINTER(C.c_int64)) for a in shp])
+        strd = (C.c_int64 * L)(*[int(v) for v in x_strides])
+        rc = self.lib.tpls_fit_batch(self.h, L, int(batch), ptrs, dts, nds, shps, strd,
+                                     _ptr(y), int(m), int(y_stride), None if row_w is None else _ptr(row_w),
+                                     int(n_components), float(tol), int(max_iter), int(flags), C.byref(out))
+        if rc == E_BATCH_UNSUPPORTED:
+            return False
+        self._ck(rc)
+        return True
 
     # ---- results ----
     def _host_out(self, rows, cols):

@@ -67,10 +67,21 @@ class ctPLS(Mapping):
         st = _core.run_fit(Xs, Y, self.n_components, tol, max_iter, device=self.device,
                            group=self.process_group, overwrite=overwrite_x, profile=profile,
                            algorithm=self.algorithm)
-        self.Xs_len = len(Xs)
-        self.Xs_dim = [X.ndim for X in Xs]
-        self.Xs_shape = [tuple(X.shape) for X in Xs]
-        self.Y_shape = (int(Y.shape[0]), 1) if Y.ndim == 1 else tuple(Y.shape)
+        self._set_fitted(st, [tuple(X.shape) for X in Xs], (int(Y.shape[0]), 1) if Y.ndim == 1 else tuple(Y.shape),
+                         [_core.weak_ref(X) for X in Xs], _core.weak_ref(Y))
+        if any(self.Xs_hasMiss):
+            print("At least one X has missing values")
+        if verbose:
+            for a, k in enumerate(self.n_iter_):
+                if self.converged_[a]:
+                    print("Comp {}: converged after {} iterations".format(a, k - 1))
+
+    def _set_fitted(self, st, Xs_shape, Y_shape, Xs_ref, Y_ref):
+        """The fitted attributes from the state of a device fit (``fit`` and ``fit_batch``)."""
+        self.Xs_len = len(Xs_shape)
+        self.Xs_dim = [len(s) for s in Xs_shape]
+        self.Xs_shape = Xs_shape
+        self.Y_shape = Y_shape
         self.factor_T = st["T"]
         # the shared score matrix is the SAME object in every tensor's factor list (cmtf.py:61-65)
         self.Xs_factors = [[self.factor_T] + ws for ws in st["W"]]
@@ -81,20 +92,14 @@ class ctPLS(Mapping):
         self.Xs_mean = st["X_mean"]
         self.Y_mean = st["Y_mean"]
         self.Xs_hasMiss = st["has_miss"]
-        if any(self.Xs_hasMiss):
-            print("At least one X has missing values")
-        self._Xs_ref = [_core.weak_ref(X) for X in Xs]   # for Xs_miss / get_q2y only; not kept alive
-        self._Y_ref = _core.weak_ref(Y)
+        self._Xs_ref = Xs_ref   # for Xs_miss / get_q2y only; not kept alive
+        self._Y_ref = Y_ref
         self.n_iter_ = st["trips"]
         # the reference is silent when max_iter is exhausted (tpls.py:79-107); here it can be asked
         self.converged_ = st["converged"]
         self.stats_ = st["stats"]
         self._profile = st["profile"]
         self._device = st["device"]
-        if verbose:
-            for a, k in enumerate(self.n_iter_):
-                if self.converged_[a]:
-                    print("Comp {}: converged after {} iterations".format(a, k - 1))
 
     @property
     def Xs_miss(self):

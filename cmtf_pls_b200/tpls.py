@@ -71,18 +71,27 @@ class tPLS(Mapping):
         st = _core.run_fit([X], Y, self.n_components, tol, max_iter, device=self.device,
                            group=self.process_group, overwrite=overwrite_x, profile=profile,
                            algorithm=self.algorithm)
-        self.X_dim = X.ndim
-        self.X_shape = tuple(X.shape)
-        self.Y_shape = (int(Y.shape[0]), 1) if Y.ndim == 1 else tuple(Y.shape)
+        self._set_fitted(st, tuple(X.shape), (int(Y.shape[0]), 1) if Y.ndim == 1 else tuple(Y.shape),
+                         _core.weak_ref(X), _core.weak_ref(Y))
+        if self.X_hasMiss:
+            print("X has missing values")
+        if verbose:
+            for a, k in enumerate(self.n_iter_):
+                if self.converged_[a]:
+                    print("Comp {}: converged after {} iterations".format(a, k - 1))
+
+    def _set_fitted(self, st, X_shape, Y_shape, X_ref, Y_ref):
+        """The fitted attributes from the state of a device fit (``fit`` and ``fit_batch``)."""
+        self.X_dim = len(X_shape)
+        self.X_shape = X_shape
+        self.Y_shape = Y_shape
         self.X_factors = [st["T"]] + st["W"][0]
         self.Y_factors = [st["U"], st["Q"]]
         self.R2X = st["R2X"][0]
         self.R2Y = st["R2Y"]
         self.X_hasMiss = st["has_miss"][0]
-        if self.X_hasMiss:
-            print("X has missing values")
-        self._X_ref = _core.weak_ref(X)   # for X_miss / get_q2y only; the caller's arrays are not kept alive
-        self._Y_ref = _core.weak_ref(Y)
+        self._X_ref = X_ref   # for X_miss / get_q2y only; the caller's arrays are not kept alive
+        self._Y_ref = Y_ref
         self.X_mean = st["X_mean"][0]
         self.Y_mean = st["Y_mean"]
         self.coef_ = st["coef"]
@@ -92,10 +101,6 @@ class tPLS(Mapping):
         self.stats_ = st["stats"]
         self._profile = st["profile"]
         self._device = st["device"]
-        if verbose:
-            for a, k in enumerate(self.n_iter_):
-                if self.converged_[a]:
-                    print("Comp {}: converged after {} iterations".format(a, k - 1))
 
     @property
     def X_miss(self):

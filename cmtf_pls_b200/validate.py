@@ -76,6 +76,9 @@ def q2y_sweep(X, Y, n_components, n_splits=5, seed=0, device=None, tol=1e-8, max
     streaming loop to rounding, several times faster), which the library
     replaces by the streaming loop on its own when there are more than 8
     responses (4 with missing values); ``"stream"`` forces the latter.
+    ``"batch"`` fits all folds of the sweep in ONE launch of the batch kernel
+    (:func:`cmtf_pls_b200.fit_batch`, one CTA per fold; same results): the
+    fastest choice for small data sets, e.g. leave-one-out.
 
     ``fold_group`` (a torch.distributed process group, or True for the default
     one) runs the sweep FOLD-PARALLEL (SURVEY.md §8e: folds are independent
@@ -94,13 +97,25 @@ def q2y_sweep(X, Y, n_components, n_splits=5, seed=0, device=None, tol=1e-8, max
         import torch.distributed as dist
         pg = None if fold_group is True else fold_group
         rank, world = dist.get_rank(pg), dist.get_world_size(pg)
-    if _fit_fold is None:                      # tests inject a CPU fit to exercise the fold plumbing without a GPU
+    mine = folds[rank::world]
+    if algorithm == "batch" and _fit_fold is None:
+        # all folds of this rank in ONE launch of the batch kernel: X and Y shared, one 0/1 weight row per fold
+        from .batch import fit_batch
+        masks = np.ones((len(mine), n))
+        for k, held in enumerate(mine):
+            masks[k, held] = 0.0
+        models = fit_batch([x[None] for x in Xs] if isinstance(X, (list, tuple)) else Xs[0][None], Y2[None], R,
+                           row_weights=masks, tol=tol, max_iter=max_iter, device=device) if mine else []
+        fits = iter([dict(T=mdl.factor_T if isinstance(X, (list, tuple)) else mdl.X_factors[0], coef=mdl.coef_,
+                          Q=mdl.Y_factors[1], Y_mean=mdl.Y_mean) for mdl in models])
+        _fit_fold = lambda w: next(fits)  # noqa: E731 -- the folds come back in the order of `mine`
+    elif _fit_fold is None:                    # tests inject a CPU fit to exercise the fold plumbing without a GPU
         Xd = [_to_device(x, device) for x in Xs]
         Yd = _to_device(Y2, device)
         _fit_fold = _device_fold_fit(Xd, Yd, R, tol, max_iter, device, algorithm)
     press = np.zeros(R)
     cv_scores = np.zeros((n, R))
-    for held in folds[rank::world]:
+    for held in mine:
         w = np.ones(n)
         w[held] = 0.0
         st = _fit_fold(w)

@@ -184,6 +184,48 @@ int tpls_transform(tpls_handle h, int n_tensors, int n_components, const void* c
 int tpls_reconstruct(tpls_handle h, int n_components, const double* scores, int64_t n, int64_t p, const double* wkron,
                      const void* mean, int mean_dtype, double* out);
 
+/* ---- batched fits: many small problems in ONE launch, one CTA per problem ----
+ *
+ * B independent tPLS / ctPLS fits (cross-validation folds, choosing the number of components, repeated seeds,
+ * one model per subgroup), each with exactly the semantics of tpls_fit (+ tpls_set_row_weights): the same
+ * statistics, centring, inner loop, stop test, regression and deflations, rounded at the same points.  The whole
+ * fit of a problem runs inside one CTA of a persistent kernel (csrc/batch.cu): no grid barrier, no host round trip
+ * and no launch per fit.  The working set of a problem lives in shared memory when it fits (~195 KB), else in the
+ * CTA's slot of a global workspace.
+ *
+ * Problem b reads tensor l at xs[l] + b * x_batch_stride[l] elements (0 = every problem shares the tensor),
+ * shaped shapes[l][0 .. ndims[l]) = (n, d1, ...) in C order; Y at y + b * y_batch_stride, (n, m) float64; row_w
+ * (batch, n) 0/1 weights or NULL.  Inputs may be host or device memory; device inputs are read where they are and
+ * never written, host inputs are staged once.  Outputs are caller-owned, host or device, leading axis = problem.
+ *
+ * Returns 0, non-zero on an invalid argument, or TPLS_E_BATCH_UNSUPPORTED -- with nothing written -- when a
+ * problem is outside the kernel's limits: more than 8 responses, more than 32 components, a rank-1 workspace
+ * above 200 KB, or a working set per problem above TPLS_BATCH_MB megabytes (default 16).  The caller then fits the
+ * problems one by one with tpls_fit.  TPLS_BATCH=0 forces that code; TPLS_BATCH_SMEM=0 keeps the working sets in
+ * global memory (both for A/B runs and tests). */
+#define TPLS_E_BATCH_UNSUPPORTED 2
+
+typedef struct tpls_batch_out {
+    double* T; double* U;             /* (B, n, R) */
+    double* Q;                        /* (B, m, R) */
+    double* W[TPLS_MAX_TENSORS];      /* (B, sum_k shape[k] for k >= 1, R): the loading matrices of modes 1.. back to back */
+    double* coef;                     /* (B, R, R) */
+    double* r2x;                      /* (B, n_tensors, R) */
+    double* r2y;                      /* (B, R) */
+    void* x_mean[TPLS_MAX_TENSORS];   /* (B, P_l) in X's dtype */
+    double* y_mean;                   /* (B, m) */
+    int* trips; int* converged;       /* (B, R) */
+    int* has_missing;                 /* (B, n_tensors) */
+    double fit_ms;                    /* out: device time of the call (staging and result copies included) */
+} tpls_batch_out;
+
+int tpls_fit_batch(tpls_handle h, int n_tensors, int64_t batch,
+                   const void* const* xs, const int* dtypes, const int* ndims, const int64_t* const* shapes,
+                   const int64_t* x_batch_stride,
+                   const double* y, int64_t m, int64_t y_batch_stride,
+                   const double* row_w,
+                   int n_components, double tol, int max_iter, int flags, tpls_batch_out* out);
+
 /* ---- single operators (used by the parity tests and by bench.py's per-kernel roofline) ----
  * All pointers here are DEVICE pointers; x is (n, p) C-ordered with p*elem a multiple of 16. */
 /* z[p] = sum_i x[i,:] * u[i]                      tpls.py:83  (masked: missingvals.py:7-20, n_total = n) */
