@@ -11,7 +11,9 @@
 //   tail         solve_coef (unit-norm score columns, dependent columns get 0), the Y deflation, the X deflation
 //                fused with its residual norm; after the last component the norm of the unrounded residual
 // Held-out rows (weight 0) are centred, projected and deflated like the others, so their scores are transform() of
-// those rows under the fold's model.
+// those rows under the fold's model.  Such a score is NaN for a row without observed entries, and deflation by it
+// turns that row of a dense coupled tensor NaN too; so every sum over rows skips a weight-0 row instead of
+// multiplying it by 0 (NaN * 0 is NaN).  On finite data the skip gives the bits of the multiply.
 #include "batch.cuh"
 #include "rank1_task.cuh"
 
@@ -142,17 +144,18 @@ __global__ void __launch_bounds__(kRank1Threads, 1) batch_fit_kernel(const __gri
                 double xd = stx(xw, dt, e, fma(-1.0, mean[c], x));  // NaN stays NaN
                 if (masked && !(x == x)) xd = 0.0;
                 const double sw = wr != nullptr ? wr[i] : 1.0;
-                ss = fma(sw * xd, xd, ss);
+                if (sw != 0.0) ss = fma(xd, xd, ss);
             }
             ss = block_sum(ss, red);
             if (tid == 0) ss_s[l * (R + 1)] = ss;
             if (masked) {
-                // observed entries per row, counted on the input (what the counting row pass reads)
+                // observed entries per row, counted after centring as transform() counts them: an entry of a column
+                // without observed training entries (NaN mean) is not observed
                 double* rowcnt = reinterpret_cast<double*>(ws + X.off_rowcnt);
                 for (int i = warp; i < n; i += NWARP) {
                     double c = 0.0;
                     for (int j = lane; j < p; j += 32) {
-                        const double v = ldx(xin, dt, (size_t)i * p + j);
+                        const double v = ldx(xw, dt, (size_t)i * p + j);
                         c += v == v ? 1.0 : 0.0;
                     }
                     c = warp_sum(c);
@@ -288,7 +291,10 @@ __global__ void __launch_bounds__(kRank1Threads, 1) batch_fit_kernel(const __gri
                 }
                 __syncthreads();
                 // q = Y't / ||Y't|| and the stop test (tpls.py:100-107)
-                col_reduce(n, M, scr, [&](int i, int c, double& s1, double&) { s1 = fma(Yw[(size_t)i * M + c], Ta[i], s1); },
+                col_reduce(n, M, scr, [&](int i, int c, double& s1, double&) {
+                               const double sw = wr != nullptr ? wr[i] : 1.0;
+                               if (sw != 0.0) s1 = fma(Yw[(size_t)i * M + c], Ta[i], s1);
+                           },
                            [&](int c, double s1, double) { qraw_s[c] = s1; });
                 if (tid == 0) {
                     double nrm = 0.0;
@@ -337,10 +343,10 @@ __global__ void __launch_bounds__(kRank1Threads, 1) batch_fit_kernel(const __gri
                 const double* pa = Tw + (size_t)(j < ka ? j : j - ka) * n;
                 const double* pb = j < ka ? Ta : uw;
                 double s = 0.0;
+#pragma unroll 1  // unrolled, this loop pushes the kernel past its 128 registers into a spill
                 for (int i = lane; i < n; i += 32) {
-                    double av = pa[i];
-                    if (wr != nullptr) av *= wr[i];
-                    s = fma(av, pb[i], s);
+                    const double sw = wr != nullptr ? wr[i] : 1.0;
+                    if (sw != 0.0) s = fma(pa[i], pb[i], s);
                 }
                 s = warp_sum(s);
                 if (lane == 0) dots_s[j] = s;
@@ -396,18 +402,15 @@ __global__ void __launch_bounds__(kRank1Threads, 1) batch_fit_kernel(const __gri
                 for (int i = tid; i < n; i += NTH) {
                     double sv = 0.0;
                     for (int b = 0; b < ka; ++b) sv = fma(Tw[(size_t)b * n + i], xs_s[b], sv);
-                    double sw = 1.0;
-                    if (wr != nullptr) {
-                        sw = wr[i];
-                        sv *= sw;
-                    }
+                    const double sw = wr != nullptr ? wr[i] : 1.0;
+                    if (sw == 0.0) continue;  // a held-out row of Y stays 0
                     double rs = 0.0;
                     for (int c = 0; c < M; ++c) {
                         const double yv = fma(-sv, q_s[c], Yw[(size_t)i * M + c]);
                         Yw[(size_t)i * M + c] = yv;
                         rs = fma(yv, yv, rs);
                     }
-                    ssy = fma(sw, rs, ssy);
+                    ssy += rs;
                 }
                 ssy = block_sum(ssy, red);
                 if (tid == 0) ssy_s[comp + 1] = ssy;
@@ -428,7 +431,7 @@ __global__ void __launch_bounds__(kRank1Threads, 1) batch_fit_kernel(const __gri
                     if (write) xd = stx(xw, dt, e, xd);  // NaN stays NaN
                     if (masked_s[l] && !(x == x)) xd = 0.0;
                     const double sw = wr != nullptr ? wr[i] : 1.0;
-                    ss = fma(sw * xd, xd, ss);
+                    if (sw != 0.0) ss = fma(xd, xd, ss);
                 }
                 ss = block_sum(ss, red);
                 if (tid == 0) ss_s[l * (R + 1) + comp + 1] = ss;

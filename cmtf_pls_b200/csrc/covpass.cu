@@ -146,7 +146,8 @@ __global__ void __launch_bounds__(kThreads, 2) covpass_kernel(const __grid_const
         if (cvalid) {
             for (int r = rl; r < rows; r += g.rpt) {
                 const long long grow = r0 + r;
-                const double ar = a.row_a != nullptr ? __ldg(a.row_a + grow) : 1.0;
+                double ar = a.row_a != nullptr ? __ldg(a.row_a + grow) : 1.0;
+                if (!(ar == ar)) ar = 0.0;  // a NaN score: leave the row as it is (see col_pass)
                 const double sw = a.row_sw != nullptr ? __ldg(a.row_sw + grow) : 1.0;
                 double yv[MR];
 #pragma unroll
@@ -158,22 +159,26 @@ __global__ void __launch_bounds__(kThreads, 2) covpass_kernel(const __grid_const
 #pragma unroll
                     for (int m = 0; m < MY; ++m) yv[MY + m] = yv[m] * sc;
                 }
+                if (sw == 0.0) {  // a held-out row adds nothing (its rescale can be inf: 0 * inf is NaN)
+#pragma unroll
+                    for (int m = 0; m < MR; ++m) yv[m] = 0.0;
+                }
                 Pack<XT> in, out;
                 in.v = *reinterpret_cast<const typename VecOf<XT>::type*>(tp + (size_t)r * srow + cl * VEC);
                 double rs = 0.0;
 #pragma unroll
                 for (int j = 0; j < VEC; ++j) {
                     const XT xs = in.e[j];
-                    const bool ob = MASKED ? (xs == xs) : true;
                     double xd = fma(-ar, wreg[j], (double)xs);
                     out.e[j] = (XT)xd;      // NaN stays NaN
                     xd = (double)out.e[j];  // later passes see the stored (rounded) value
+                    const bool ob = MASKED ? (xd == xd) : true;  // observed after centring (NaN mean: missing)
                     if (MASKED && !ob) xd = 0.0;
 #pragma unroll
                     for (int m = 0; m < MR; ++m) acc[j][m] = fma(xd, yv[m], acc[j][m]);
                     rs = fma(xd, xd, rs);
                 }
-                ss = fma(sw, rs, ss);
+                if (sw != 0.0) ss = fma(sw, rs, ss);
                 __stcs(reinterpret_cast<typename VecOf<XT>::type*>(xo + grow * g.pitch + c0 + cl * VEC), out.v);
             }
         }

@@ -840,12 +840,14 @@ static void r1_config(tpls_handle h, int L, size_t* r1_smem, bool* r1_use_smem) 
     }
 }
 
-// observed entries per row of a masked tensor (constant during the fit): one counting row pass with zero weights
+// observed entries per row of a masked tensor after centring (constant during the fit): one counting row pass over
+// the input with the column means as weights; an entry of a column whose mean is NaN does not count.  Its
+// projection, into the scratch vector, is not used.
 static int count_rows(tpls_handle h, Tensor& t) {
     RowPassArgs r{};
     r.g = t.gr_cnt;
     r.x_in = t.src;
-    r.col_w = t.wkron;  // still all zero
+    r.col_w = t.mean_d;
     r.t_out = h->svec;
     r.tpart = t.tpart;
     r.cpart = t.cpart;

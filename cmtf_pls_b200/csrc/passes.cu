@@ -167,6 +167,9 @@ __global__ void __launch_bounds__(kThreads, 2) colpass_kernel(const __grid_const
             const long long grow = r0 + r;
             double ar = 1.0, ur = 0.0;
             if (DEFLATE && a.row_a != nullptr) ar = __ldg(a.row_a + grow);
+            // a NaN score: the row has a tensor without observed entries, so its later scores are NaN whatever it
+            // holds; left as it is, it keeps NaN out of the sums over rows (NaN * 0 is NaN)
+            if (DEFLATE && !(ar == ar)) ar = 0.0;
             if (CONTRACT) {
                 if (use_y) {
                     // (a compile-time unrolled variant with two chains was measured against this loop on one box:
@@ -197,7 +200,6 @@ __global__ void __launch_bounds__(kThreads, 2) colpass_kernel(const __grid_const
 #pragma unroll
                 for (int j = 0; j < VEC; ++j) {
                     const XT xs = in.e[j];
-                    const bool ob = MASKED ? (xs == xs) : true;
                     double xd = (double)xs;
                     if (DEFLATE) {
                         xd = fma(-ar, wreg[k][j], xd);
@@ -210,6 +212,9 @@ __global__ void __launch_bounds__(kThreads, 2) colpass_kernel(const __grid_const
                         // stored values by ~6e-8 / sqrt(elements) relative, and saves two of its three conversions
                         // per element, which are what bounds it)
                     }
+                    // observed after centring, as transform() counts: an entry of a column whose mean is NaN (no
+                    // observed training entry) is missing
+                    const bool ob = MASKED ? (xd == xd) : true;
                     if (MASKED && !ob) xd = 0.0;
                     if (CONTRACT) zacc[k][j] = fma(xd, ur, zacc[k][j]);
                     if (COLSTAT) {
@@ -224,7 +229,7 @@ __global__ void __launch_bounds__(kThreads, 2) colpass_kernel(const __grid_const
                 }
             }
             if (SUMSQ) {
-                ss = fma(sw, rs[0] + rs[1], ss);
+                if (sw != 0.0) ss = fma(sw, rs[0] + rs[1], ss);  // a held-out row adds nothing, even a NaN
             }
         }
         __syncwarp();
@@ -390,7 +395,10 @@ __global__ void __launch_bounds__(256) row_finish_kernel(const RowFinishArgs a) 
         if (a.qpart != nullptr) {
 #pragma unroll
             for (int m = 0; m < kMaxFusedResp; ++m)
-                if (m < a.pitch_y) qacc[m] = fma(a.y[r * a.pitch_y + m], nv, qacc[m]);
+                if (m < a.pitch_y) {
+                    const double y = a.y[r * a.pitch_y + m];
+                    if (y != 0.0) qacc[m] = fma(y, nv, qacc[m]);  // a held-out row (Y row 0) adds nothing, even a NaN t
+                }
         }
     }
     if (a.d2part != nullptr) {

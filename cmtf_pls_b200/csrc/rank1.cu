@@ -511,7 +511,10 @@ __device__ __forceinline__ void resident_project_rows(const ResidentArgs& a, int
             double ti = tl[i] + td[i];
             if (L > 1) ti = pow2 ? ti * inv_l : ti / (double)L;
             if (lane == 0) a.t_out[r_lo + k] = ti;
-            if (lane < a.pitch_y) qacc = fma(ysrc.row(k)[lane], ti, qacc);
+            if (lane < a.pitch_y) {
+                const double y = ysrc.row(k)[lane];
+                if (y != 0.0) qacc = fma(y, ti, qacc);  // a held-out row (Y row 0) adds nothing, even a NaN t
+            }
         }
     }
 }
@@ -841,7 +844,10 @@ __global__ void __launch_bounds__(kRank1Threads, 1) resident_loop_kernel(const _
             double sacc = 0.0;
             for (int k = lane; k < nblk; k += 32) {
                 double av = pa[k];
-                if (a.row_w != nullptr) av *= a.row_w[r_lo + k];
+                if (a.row_w != nullptr) {
+                    if (a.row_w[r_lo + k] == 0.0) continue;  // a held-out score can be NaN: skip, not * 0
+                    av *= a.row_w[r_lo + k];
+                }
                 sacc = fma(av, pb[k], sacc);
             }
             sacc = warp_sum(sacc);
@@ -943,6 +949,7 @@ __global__ void __launch_bounds__(kRank1Threads, 1) resident_loop_kernel(const _
             double sw = 1.0;
             if (a.row_w != nullptr) {
                 sw = a.row_w[r];
+                if (sw == 0.0) continue;  // a held-out row of Y stays 0 (its score can be NaN)
                 sv *= sw;
             }
             double* yr = a.y_rw + (size_t)r * a.pitch_y;

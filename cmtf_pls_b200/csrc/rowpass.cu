@@ -110,7 +110,8 @@ __device__ __forceinline__ double row_epilogue(const RowPassArgs& a, long long g
 // q = Y't fused into the projection (tpls.py:100): qacc[m] += Y[row, m] * t[row] for the row's FINAL t
 __device__ __forceinline__ void q_accumulate(double (&qacc)[kMaxFusedResp], const double (&yv)[kMaxFusedResp], double t) {
 #pragma unroll
-    for (int m = 0; m < kMaxFusedResp; ++m) qacc[m] = fma(yv[m], t, qacc[m]);
+    for (int m = 0; m < kMaxFusedResp; ++m)
+        if (yv[m] != 0.0) qacc[m] = fma(yv[m], t, qacc[m]);  // a held-out row (Y row 0) adds nothing, even a NaN t
 }
 
 __device__ __forceinline__ void load_y_row(const RowPassArgs& a, long long grow, double (&yv)[kMaxFusedResp]) {
@@ -383,7 +384,9 @@ __global__ void __launch_bounds__(kRowThreads, 2) rowpass_kernel(const __grid_co
                                 const bool ob = (xs == xs);
                                 const XT xc = ob ? xs : (XT)0;  // select in the storage type, convert once
                                 acc[k][j] = (double)xc * wreg[k][j];
-                                if (COUNT) icnt += (ob && (FULL || cvalid[k])) ? 1 : 0;
+                                // counting: the weights are the column means, and an entry of a column whose mean is
+                                // NaN (no observed training entry) is missing after centring, as transform() counts
+                                if (COUNT) icnt += (ob && wreg[k][j] == wreg[k][j] && (FULL || cvalid[k])) ? 1 : 0;
                             } else {
                                 acc[k][j] = (double)xs * wreg[k][j];
                             }

@@ -153,7 +153,7 @@ __global__ void __launch_bounds__(256) multi_dot_kernel(const __grid_constant__ 
     const double* b = d.b[j];
     double s = 0.0;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < d.n; i += (long long)gridDim.x * blockDim.x)
-        s = fma(d.w != nullptr ? a[i] * d.w[i] : a[i], b[i], s);
+        if (d.w == nullptr || d.w[i] != 0.0) s = fma(d.w != nullptr ? a[i] * d.w[i] : a[i], b[i], s);  // NaN * 0 is NaN
     s = block_sum(s, red);
     if (threadIdx.x == 0) part[(size_t)blockIdx.x * d.npairs + j] = s;
 }
@@ -231,7 +231,7 @@ __global__ void lincomb_kernel(const double* T, long long n, long long ldt, cons
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
         double s = 0.0;
         for (int b = 0; b <= a; ++b) s = fma(T[b * ldt + i], coef[b * R + a], s);
-        out[i] = row_w != nullptr ? s * row_w[i] : s;
+        out[i] = row_w == nullptr ? s : (row_w[i] != 0.0 ? s * row_w[i] : 0.0);  // a NaN score of a held-out row
     }
 }
 
